@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DynaBOA per-frame hot path: adapted frames/sec on the synthetic 3DPW-shape stream.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c5] [--dump-outputs DIR]
 
 One "step" = one adapted frame at BASELINE.json configs[1] (C2: 1 inner step, batch 1; S-adapt scope of
 SURVEY.md §8d: adaptation + one output forward/SMPL).  Prints ONE JSON line (see DESIGN.md "Measurement").
@@ -178,7 +178,7 @@ def time_oracle(workload, steps, warmup):
 
 def time_reference_code(workload, steps, warmup):
     """The reference's OWN CPU implementation (oracle/ref_harness.py: model/hmr.py, base_adaptor.py, dynaboa_benchmark.Adaptor from
-    /root/reference or its copy baseline/_ref, unmodified; smplx / learn2learn restated, synthetic stream), S-adapt scope:
+    the checkout named by DBOA_REFERENCE_ROOT or the bytecode build() made of it under oracle/_ref, unmodified; smplx / learn2learn restated, synthetic stream), S-adapt scope:
     ``Adaptor.adaptation`` evaluates the model after every inner step and after the outer step (two ``inference`` calls per frame
     in C2), the GPU arm runs ONE output forward per frame -- the time of all but the last ``inference`` call of a frame is
     measured by a wrapper and subtracted.  Returns (frames/s, seconds, description) or None when the reference tree is absent."""
@@ -218,7 +218,7 @@ def time_reference_code(workload, steps, warmup):
             if t >= warmup:
                 times.append(dt)
     shutil.rmtree(work, ignore_errors=True)
-    root = 'baseline/_ref' if 'baseline' in ref_harness.REF else ref_harness.REF
+    root = 'oracle/_ref' if ref_harness.REF == ref_harness.BUILT else ref_harness.REF
     return 1.0 / float(np.median(times)), float(np.sum(times)), f'unmodified reference code from {root} (oracle/ref_harness.py)'
 
 
@@ -266,6 +266,14 @@ def run_reference(args, rank, world):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
+def dump_outputs(out_dir, outputs):
+    """What the caller of the timed path receives for the last timed frame (rotmat, betas, cam, joints, vertices: ~110 KB), as
+    ``<out_dir>/<name>.npy`` in float32, so that two builds can be compared output for output on the same seeded stream."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in outputs.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), v.detach().float().cpu().numpy())
+
+
 def run_ours(args, rank, world, local):
     from dynaboa_b200 import _lib, config, dist as ddist, hmr as hmr_mod, synthetic
     from dynaboa_b200.adaptor import Adaptor
@@ -354,7 +362,7 @@ def run_ours(args, rank, world, local):
             e0.record()
             marks = []
             for t in range(PRELUDE + args.warmup, n_frames):
-                step(t, from_host)
+                pred = step(t, from_host)
                 if args.frame_times:                     # diagnostic: one event per frame on the adaptation stream
                     marks.append(torch.cuda.Event(enable_timing=True))
                     marks[-1].record()
@@ -371,7 +379,7 @@ def run_ours(args, rank, world, local):
                              f' | drain {ms - ts[-1]:.2f}\n')
         launches = lib.dboa_launch_count() - l0
         clocks = sampler.stop() if sampler else None
-        return ddist.max_over_ranks(ms, dev), launches, clocks
+        return ddist.max_over_ranks(ms, dev), launches, clocks, pred
 
     # reset model state between the two measurements so both see the same trajectory
     snapshot = (ad.model.module.arena.clone(), ad.teacher.arena.clone())
@@ -381,10 +389,12 @@ def run_ours(args, rank, world, local):
         ad.optimizer.m.zero_(); ad.optimizer.v.zero_(); ad.optimizer.step_count = 0
 
     sys.stderr.write('[bench] setup done\n')
-    ms_dev, launches, clocks = timed(False)
+    ms_dev, launches, clocks, last = timed(False)
     sys.stderr.write(f'[bench] device-resident: {ms_dev / args.steps:.2f} ms/frame\n')
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     restore()
-    ms_e2e, _, clocks_e2e = timed(True)
+    ms_e2e, _, clocks_e2e, _ = timed(True)
     value = world * args.steps / (ms_dev / 1000.0)
     e2e = world * args.steps / (ms_e2e / 1000.0)
 
@@ -466,7 +476,13 @@ def main():
     ap.add_argument('--serial-output', action='store_true',
                     help='run the output forward on the adaptation stream (no overlap with the next frame)')
     ap.add_argument('--tc', type=int, default=-1, help='tensor-core conv mode override (0 fp32 CUDA cores, 1 forward, 2 forward+dgrad+wgrad, 3 forward+dgrad)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the outputs of the last timed frame as DIR/<name>.npy (rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to the GPU path (--impl ours)')
     if args.warmup < 3 and args.impl == 'ours':
         args.warmup = 3
     from dynaboa_b200 import dist as ddist

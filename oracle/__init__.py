@@ -19,9 +19,8 @@ algorithm of the reference's per-frame hot path (SURVEY.md §8):
 Pinning status (see DESIGN.md "Oracle"):
 
 * geometry / prior / hmr restatements are checked bit-for-bit against the reference's own
-  modules imported from /root/reference by ``oracle/make_golden.py`` (run in the build
-  container, where the reference is mounted), and the resulting vectors are committed under
-  ``tests/golden/``.
+  modules imported from the checkout named by DBOA_REFERENCE_ROOT by ``oracle/make_golden.py``,
+  and the resulting vectors are committed under ``tests/golden/``.
 * the loss assembly and the adaptation orchestration are checked against the reference's own
   ``base_adaptor.BaseAdaptor`` / ``dynaboa_benchmark.Adaptor`` code executed on CPU with the two
   missing third-party packages replaced by the restatements here.

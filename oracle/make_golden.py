@@ -1,6 +1,6 @@
-"""Golden-vector generator (run in the BUILD CONTAINER, where /root/reference is mounted).
+"""Golden-vector generator (run where a checkout of the reference is at hand).
 
-    python -m oracle.make_golden            # writes tests/golden/*.npz
+    DBOA_REFERENCE_ROOT=/path/to/DynaBOA python -m oracle.make_golden [name ...]      # writes tests/golden/*.npz
 
 What it does (test infrastructure only; nothing here ships or runs on the GPU box):
 
@@ -12,9 +12,11 @@ What it does (test infrastructure only; nothing here ships or runs on the GPU bo
    ``dynaboa_benchmark.Adaptor.adaptation`` / ``inference`` UNMODIFIED on CPU -- the two missing
    third-party packages (smplx, learn2learn) and the viz-only imports are replaced by the
    restatements/stubs below, ``__init__``'s file loading is replaced by the synthetic assets --
-   asserts ``oracle/adaptor_ref.py`` reproduces the trajectory, and stores it as fixtures.
+   asserts ``oracle/adaptor_ref.py`` reproduces the trajectory, and stores it as fixtures;
+3. records which names the reference driver ``dynaboa_benchmark.py`` takes from ``self`` and which modules it imports
+   (``driver_surface.npz``), the interface the drop-in tree has to provide.
 
-The reference is read from /root/reference at run time and never copied.
+The reference is read from DBOA_REFERENCE_ROOT at run time and never copied.
 """
 import importlib
 import importlib.util
@@ -29,7 +31,7 @@ import numpy as np
 import torch
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = '/root/reference'
+REF = os.environ.get('DBOA_REFERENCE_ROOT')
 OUT = os.path.join(REPO, 'tests', 'golden')
 sys.path.insert(0, REPO)
 
@@ -526,7 +528,30 @@ def golden_webcam(workdir, n_frames=6):
     print('adapt webcam ok')
 
 
+# ---------------------------------------------------------------------------------------
+# part 4: the interface of the unchanged driver (read from its syntax tree, never executed)
+# ---------------------------------------------------------------------------------------
+def golden_driver_surface():
+    import ast
+    tree = ast.parse(open(os.path.join(REF, 'dynaboa_benchmark.py')).read())
+    used, assigned = set(), set()
+    for node in ast.walk(tree):
+        if isinstance(node, ast.Attribute) and isinstance(node.value, ast.Name) and node.value.id == 'self':
+            (assigned if isinstance(node.ctx, ast.Store) else used).add(node.attr)
+    methods = {n.name for c in tree.body if isinstance(c, ast.ClassDef) for n in c.body if isinstance(n, ast.FunctionDef)}
+    imports = set()
+    for node in tree.body:
+        if isinstance(node, ast.ImportFrom):
+            imports.add(node.module)
+        elif isinstance(node, ast.Import):
+            imports.update(a.name for a in node.names)
+    names = dict(self_used=used, self_assigned=assigned, driver_methods=methods, imports=imports)
+    np.savez_compressed(os.path.join(OUT, 'driver_surface.npz'), **{k: np.array(sorted(v), dtype=str) for k, v in names.items()})
+    print('driver_surface.npz', {k: len(v) for k, v in names.items()})
+
+
 def main():
+    assert REF and os.path.isdir(REF), 'set DBOA_REFERENCE_ROOT to a checkout of the reference'
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(os.cpu_count())
     workdir = tempfile.mkdtemp(prefix='dboa_golden_')
@@ -534,7 +559,9 @@ def main():
         synthetic.write_asset_dir(os.path.join(workdir, 'data'))
         os.makedirs(os.path.join(workdir, 'data/spin_data'), exist_ok=True)
         os.symlink(os.path.join(REF, 'data/gmm_08.pkl'), os.path.join(workdir, 'data/spin_data/gmm_08.pkl'))
-        which = sys.argv[1:] or ['geometry', 'prior', 'hmr', 'smpl', 'eval', 'c2', 'c3', 'c5', 'dp2', 'dataprocess', 'webcam']
+        which = sys.argv[1:] or ['geometry', 'prior', 'hmr', 'smpl', 'eval', 'c2', 'c3', 'c5', 'dp2', 'dataprocess', 'webcam', 'surface']
+        if 'surface' in which:
+            golden_driver_surface()
         if 'dp2' in which:
             golden_dp()
         if 'dataprocess' in which:

@@ -1,8 +1,8 @@
 """The reference's OWN adaptor code on CPU (test / benchmark infrastructure only; never imported by the product).
 
-``make_reference_adaptor`` builds ``dynaboa_benchmark.Adaptor`` from the reference tree -- ``/root/reference`` in the build
-container, the byte-for-byte copy ``baseline/_ref/`` (scripts/install_reference.py, git-ignored, travels with gpurun) on the GPU
-box -- with the constructor's I/O replaced: the two third-party packages that are not in this image (``smplx``,
+``make_reference_adaptor`` builds ``dynaboa_benchmark.Adaptor`` from the reference tree -- a checkout named by
+``DBOA_REFERENCE_ROOT``, else the bytecode build() made under the git-ignored ``oracle/_ref/`` (oracle/build_ref.py) -- with the
+constructor's I/O replaced: the two third-party packages that are not in this image (``smplx``,
 ``learn2learn``) are the restatements of this package, the datasets are the synthetic stream / exemplar bank, the device is the
 CPU.  Everything that runs per frame -- ``model/hmr.py``, ``base_adaptor.BaseAdaptor``'s losses and levels,
 ``dynaboa_benchmark.Adaptor.adaptation`` / ``inference``, ``utils/geometry.py``, ``utils/smplify/prior.py``,
@@ -21,16 +21,27 @@ from dynaboa_b200 import constants as C
 from dynaboa_b200 import synthetic
 from . import adaptor_ref, l2l_ref, smplx_ref
 
-REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+BUILT = os.path.join(os.path.dirname(os.path.abspath(__file__)), '_ref')      # made by build() (oracle/build_ref.py)
+
+
+def _module_file(root, name):
+    """``<root>/<name>.py``, or its bytecode ``<root>/<name>.pyc`` (the form under oracle/_ref); None when neither exists."""
+    for ext in ('.py', '.pyc'):
+        path = os.path.join(root, name + ext)
+        if os.path.exists(path):
+            return path
+    return None
 
 
 def reference_root():
-    """/root/reference when present (build container), else the copy under baseline/_ref, else None
-    (DBOA_REFERENCE_ROOT overrides; ``none`` disables the reference tree: the callers fall back to the oracle port)."""
-    if os.environ.get('DBOA_REFERENCE_ROOT') == 'none':
+    """The reference checkout named by DBOA_REFERENCE_ROOT, else the reference files build() compiled into oracle/_ref/, else
+    None (``DBOA_REFERENCE_ROOT=none`` disables both): the callers then fall back to the oracle port or skip."""
+    env = os.environ.get('DBOA_REFERENCE_ROOT')
+    if env == 'none':
         return None
-    for root in (os.environ.get('DBOA_REFERENCE_ROOT'), '/root/reference', os.path.join(REPO, 'baseline', '_ref')):
-        if root and os.path.exists(os.path.join(root, 'dynaboa_benchmark.py')) and os.path.exists(os.path.join(root, 'model', 'hmr.py')):
+    for root in (env, BUILT):
+        if root and _module_file(root, 'dynaboa_benchmark') and _module_file(root, os.path.join('model', 'hmr')):
             return root
     return None
 
@@ -40,6 +51,11 @@ REF = reference_root()
 
 def available():
     return REF is not None
+
+
+def driver(name):
+    """Path of the reference's driver script ``name`` (``dynaboa_benchmark``, ``dynaboa_internet``), or None."""
+    return _module_file(REF, name) if REF else None
 
 
 class _StubSMPLX(torch.nn.Module):

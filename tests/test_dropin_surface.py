@@ -1,25 +1,17 @@
 """Static check of the drop-in boundary (SURVEY.md §8b): every attribute / method the UNCHANGED reference
 driver touches on ``self`` exists on our BaseAdaptor (or is created by the driver itself), and every module it
-imports resolves inside dynaboa_b200/dropin.  Needs the reference checkout, so it only runs in the build
-container; it never executes the reference."""
+imports resolves inside dynaboa_b200/dropin.  The driver's side of the boundary is the fixture
+tests/golden/driver_surface.npz, read from its syntax tree by oracle/make_golden.py; the reference is never executed."""
 import ast
 import os
 import sys
 
-import pytest
-
-REF = '/root/reference/dynaboa_benchmark.py'
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason='reference checkout not present (GPU box)')
-def test_driver_surface_is_provided():
-    tree = ast.parse(open(REF).read())
-    used, assigned = set(), set()
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Attribute) and isinstance(node.value, ast.Name) and node.value.id == 'self':
-            (assigned if isinstance(node.ctx, ast.Store) else used).add(node.attr)
-    driver_methods = {n.name for c in tree.body if isinstance(c, ast.ClassDef) for n in c.body if isinstance(n, ast.FunctionDef)}
+def test_driver_surface_is_provided(golden):
+    ref = golden('driver_surface')
+    used, assigned, driver_methods = ({str(s) for s in ref[k]} for k in ('self_used', 'self_assigned', 'driver_methods'))
     src = open(os.path.join(REPO, 'dynaboa_b200', 'base_adaptor.py')).read()
     base = ast.parse(src)
     provided = {n.name for c in base.body if isinstance(c, ast.ClassDef) and c.name == 'BaseAdaptor' for n in c.body
@@ -31,17 +23,11 @@ def test_driver_surface_is_provided():
     missing = used - assigned - driver_methods - provided - dead
     assert not missing, f'reference driver uses self.{sorted(missing)} which BaseAdaptor does not provide'
     dropin = os.path.join(REPO, 'dynaboa_b200', 'dropin')
-    for node in tree.body:
-        mods = []
-        if isinstance(node, ast.ImportFrom):
-            mods = [node.module]
-        elif isinstance(node, ast.Import):
-            mods = [a.name for a in node.names]
-        for m in mods:
-            top = m.split('.')[0]
-            if top in ('constants', 'utils', 'base_adaptor', 'model', 'config', 'boa_dataset'):
-                path = os.path.join(dropin, *m.split('.'))
-                assert os.path.exists(path + '.py') or os.path.isdir(path), f'drop-in tree lacks module {m}'
+    for m in (str(s) for s in ref['imports']):
+        top = m.split('.')[0]
+        if top in ('constants', 'utils', 'base_adaptor', 'model', 'config', 'boa_dataset'):
+            path = os.path.join(dropin, *m.split('.'))
+            assert os.path.exists(path + '.py') or os.path.isdir(path), f'drop-in tree lacks module {m}'
 
 
 def test_dropin_modules_import_without_gpu():

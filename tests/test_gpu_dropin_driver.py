@@ -1,7 +1,8 @@
-"""The UNCHANGED reference driver (`dynaboa_benchmark.py`, copied byte for byte into the git-ignored baseline/_ref/ by
-scripts/install_reference.py) executed on the GPU on top of the drop-in module tree, against the trajectory the
-reference itself produced on CPU (tests/golden/adapt_c2.npz, recorded by oracle/make_golden.py from the same file).
-This is the north-star claim "dynaboa_benchmark.py drops in unchanged", run rather than AST-checked."""
+"""The UNCHANGED reference driver (`dynaboa_benchmark.py`, compiled by build() into the git-ignored oracle/_ref/ --
+oracle/build_ref.py -- or taken from the checkout named by DBOA_REFERENCE_ROOT) executed on the GPU on top of the drop-in module
+tree, against the trajectory the reference itself produced on CPU (tests/golden/adapt_c2.npz, recorded by
+oracle/make_golden.py from the same file).  This is the north-star claim "dynaboa_benchmark.py drops in unchanged", run
+rather than AST-checked (tests/test_dropin_surface.py checks the interface without the reference)."""
 import os
 import runpy
 import sys
@@ -11,14 +12,15 @@ import pytest
 import torch
 
 from conftest import rel_err
+from oracle import ref_harness
 
 pytestmark = pytest.mark.gpu
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-DRIVER = os.path.join(REPO, 'baseline', '_ref', 'dynaboa_benchmark.py')
+DRIVER = ref_harness.driver('dynaboa_benchmark')
 SHADOWED = ('constants', 'config', 'model', 'utils', 'base_adaptor', 'boa_dataset', 'learn2learn')
 
 
-@pytest.mark.skipif(not os.path.exists(DRIVER), reason='baseline/_ref/dynaboa_benchmark.py absent: run scripts/install_reference.py in the build container')
+@pytest.mark.skipif(DRIVER is None, reason='no reference driver: build() makes oracle/_ref/ where a reference checkout is readable')
 def test_unchanged_reference_driver_follows_reference_trajectory(asset_dir, tmp_path, golden, monkeypatch):
     import joblib
     from dynaboa_b200 import hmr as hmr_mod

@@ -1,7 +1,8 @@
-"""Second client of the hot path (N3): the UNCHANGED reference `dynaboa_internet.py` (baseline/_ref/, byte-for-byte copy) on the
-drop-in tree, fed by a small synthetic "Internet video" on disk (PNG frames + the reference's npz annotation layout) whose crops
-and keypoints go through the GPU input side (N2), against the CPU oracle run on the oracle-processed frames.  Also the
-library's own ``InternetAdaptor`` (autograd and fused paths)."""
+"""Second client of the hot path (N3): the UNCHANGED reference `dynaboa_internet.py` (compiled by build() into the git-ignored
+oracle/_ref/ -- oracle/build_ref.py -- or taken from the checkout named by DBOA_REFERENCE_ROOT) on the drop-in tree, fed by
+a small synthetic "Internet video" on disk (PNG frames + the reference's npz annotation layout) whose crops and keypoints go
+through the GPU input side (N2), against the CPU oracle run on the oracle-processed frames.  Also the library's own
+``InternetAdaptor`` (autograd and fused paths)."""
 import os
 import runpy
 import sys
@@ -12,10 +13,11 @@ import pytest
 import torch
 
 from conftest import rel_err
+from oracle import ref_harness
 
 pytestmark = pytest.mark.gpu
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-DRIVER = os.path.join(REPO, 'baseline', '_ref', 'dynaboa_internet.py')
+DRIVER = ref_harness.driver('dynaboa_internet')
 SHADOWED = ('constants', 'config', 'model', 'utils', 'base_adaptor', 'boa_dataset', 'learn2learn')
 FLAGS = dict(inner_step=1, retrieval=0, lower_level_mixtrain=0, upper_level_mixtrain=0, dynamic_boa=0)
 N = 3
@@ -63,7 +65,7 @@ def oracle_trajectory(frames, centers, scales, parts, masks):
     return preds
 
 
-@pytest.mark.skipif(not os.path.exists(DRIVER), reason='baseline/_ref/dynaboa_internet.py absent: run scripts/install_reference.py in the build container')
+@pytest.mark.skipif(DRIVER is None, reason='no reference driver: build() makes oracle/_ref/ where a reference checkout is readable')
 def test_unchanged_internet_driver_on_gpu_input_side(asset_dir, tmp_path, monkeypatch):
     import joblib
     from dynaboa_b200 import config, hmr as hmr_mod
