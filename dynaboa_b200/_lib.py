@@ -48,6 +48,8 @@ SIGNATURES = {
     'dboa_get_fused_forward': (I, []),
     'dboa_set_fused_backward': (I, [I]),
     'dboa_set_forward_cta_budget': (I, [I]),
+    'dboa_set_split_limits': (I, [I, I, I, I]),
+    'dboa_last_wide_plan': (I, [I, C.POINTER(L)]),
     'dboa_set_operand_tmem': (I, [I]),
     'dboa_get_operand_tmem': (I, []),
     'dboa_set_chain_flags': (I, [I]),

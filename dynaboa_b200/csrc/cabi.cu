@@ -77,6 +77,18 @@ int dboa_set_fused_forward(int enable) { hmr_set_fused_forward(enable != 0); ret
 int dboa_get_fused_forward(void) { return hmr_fused_forward() ? 1 : 0; }
 int dboa_set_fused_backward(int enable) { hmr_set_fused_backward(enable != 0); return DBOA_OK; }
 int dboa_set_forward_cta_budget(int n) { conv_wide_set_cta_budget(n < 0 ? 0 : n); return DBOA_OK; }
+int dboa_set_split_limits(int kernel, int max_ctas, int max_nz, int min_kb) {
+    switch (kernel) {
+        case 0: conv_wide_set_limits(max_ctas, max_nz, min_kb); return DBOA_OK;
+        case 1: dgrad_wide_set_limits(max_ctas, max_nz, min_kb); return DBOA_OK;
+        case 2: conv_wgrad_wide_set_limits(max_ctas, max_nz, min_kb); return DBOA_OK;
+        default: return DBOA_ERR_ARG;
+    }
+}
+int dboa_last_wide_plan(int kernel, long long out[5]) {
+    if (!out) return DBOA_ERR_ARG;
+    return wide_plan_last(kernel, out) ? DBOA_OK : DBOA_ERR_ARG;
+}
 int dboa_set_operand_tmem(int enable) { conv_wide_set_operand_tmem(enable != 0); return DBOA_OK; }
 int dboa_selftest_map_cache(int bound, int n, int window) { return map_cache_selftest(bound, n, window); }
 int dboa_set_chain_flags(int enable) { hmr_set_chain_flags(enable != 0); return DBOA_OK; }

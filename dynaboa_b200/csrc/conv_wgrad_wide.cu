@@ -40,6 +40,7 @@ constexpr int NTW = 16, NTT = NTW * 32, W_MMA = 16, W_TMA = 17, NT = 576;
 constexpr uint32_t ATOM = KB * 128;                     // one box: 56 pixels x 32 channels (7168 B = 7 x 1024)
 constexpr uint32_t A_BYTES = 4 * ATOM, B_BYTES = 2 * ATOM, STAGE = A_BYTES + B_BYTES;        // 43008 B raw per stage (+ the same for lo)
 constexpr int RED_LD = BN + 4;
+constexpr int NACC = 4;                                 // TMEM accumulators a reduction chain rotates over (see conv_wide.cu)
 
 struct Launch {
     float* dw;
@@ -160,7 +161,7 @@ __global__ void __launch_bounds__(NT, 1) conv_wgrad_wide_kernel(const __grid_con
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(BN) : "memory");
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(BN * NACC) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -198,13 +199,16 @@ __global__ void __launch_bounds__(NT, 1) conv_wgrad_wide_kernel(const __grid_con
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint64_t so = (uint64_t)(st * (STAGE >> 4));
                 const uint64_t dah = draw + so, dbh = dah + (A_BYTES >> 4), dal = dlo + so, dbl = dal + (A_BYTES >> 4);
-                const uint32_t first = it > 0 ? 1u : 0u;
+                // the tensor core accumulates with truncation: k-block `it` goes to accumulator it % NACC, which keeps each chain
+                // short (one chain of 112 k-blocks was 5e-5 off an fp64 reference on a B200); the epilogue adds the accumulators in fp32
+                const uint32_t dacc = tmem_d + (uint32_t)((it & (NACC - 1)) * BN);
+                const uint32_t first = it >= NACC ? 1u : 0u;
                 if (elect_one()) {
 #pragma unroll
                     for (int kk = 0; kk < KB / 8; ++kk) {
-                        mma_tf32(tmem_d, dah + kk * KSTEP, dbh + kk * KSTEP, idesc, kk > 0 ? 1u : first);
-                        mma_tf32(tmem_d, dah + kk * KSTEP, dbl + kk * KSTEP, idesc, 1u);
-                        mma_tf32(tmem_d, dal + kk * KSTEP, dbh + kk * KSTEP, idesc, 1u);
+                        mma_tf32(dacc, dah + kk * KSTEP, dbh + kk * KSTEP, idesc, kk > 0 ? 1u : first);
+                        mma_tf32(dacc, dah + kk * KSTEP, dbl + kk * KSTEP, idesc, 1u);
+                        mma_tf32(dacc, dal + kk * KSTEP, dbh + kk * KSTEP, idesc, 1u);
                     }
                     umma_commit(&s_empty[st]);
                 }
@@ -244,9 +248,14 @@ __global__ void __launch_bounds__(NT, 1) conv_wgrad_wide_kernel(const __grid_con
     // ---- epilogue: TMEM (lane = output channel, column = input channel) -> shared memory -> cluster reduction -> dW +=
     if (warp < NTW) {
         const int q4 = warp & 3, cgp = warp >> 2;
-        uint32_t v[16];
-        if (nkb > 0) {
-            const uint32_t taddr = tmem_d + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(cgp * 16);
+        float facc[16];
+#pragma unroll
+        for (int q = 0; q < 16; ++q) facc[q] = 0.f;
+        const int nacc = nkb < NACC ? nkb : NACC;
+#pragma unroll 1
+        for (int a = 0; a < nacc; ++a) {
+            uint32_t v[16];
+            const uint32_t taddr = tmem_d + ((uint32_t)(q4 * 32) << 16) + (uint32_t)(a * BN + cgp * 16);
             asm volatile(
                 "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
                 "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
@@ -255,15 +264,12 @@ __global__ void __launch_bounds__(NT, 1) conv_wgrad_wide_kernel(const __grid_con
                 : "r"(taddr)
                 : "memory");
             asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        } else {
 #pragma unroll
-            for (int q = 0; q < 16; ++q) v[q] = 0u;
+            for (int q = 0; q < 16; ++q) facc[q] += __uint_as_float(v[q]);
         }
         const uint32_t dst = smem_u32(red) + (uint32_t)((q4 * 32 + lane) * RED_LD + cgp * 16) * 4u;
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
-            sts128(dst + q * 16, make_float4(__uint_as_float(v[q * 4]), __uint_as_float(v[q * 4 + 1]), __uint_as_float(v[q * 4 + 2]),
-                                             __uint_as_float(v[q * 4 + 3])));
+        for (int q = 0; q < 4; ++q) sts128(dst + q * 16, make_float4(facc[q * 4], facc[q * 4 + 1], facc[q * 4 + 2], facc[q * 4 + 3]));
     }
     cg::cluster_group cluster = cg::this_cluster();
     if (nz == 1) __syncthreads(); else cluster.sync();
@@ -299,7 +305,7 @@ __global__ void __launch_bounds__(NT, 1) conv_wgrad_wide_kernel(const __grid_con
     if (nz > 1) cluster.sync();
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "n"(BN) : "memory");
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "n"(BN * NACC) : "memory");
 }
 
 }  // namespace wg
@@ -308,6 +314,21 @@ bool conv_wgrad_wide_ok(const ConvDims& d) {
     const int W = d.Wo;
     return (d.stride == 1 || d.stride == 2) && d.Hi == d.Ho * d.stride && d.Wi == d.Wo * d.stride && d.Ho == d.Wo && d.Cout % 128 == 0 && d.Cin % 64 == 0 && (d.kh == 1 || d.kh == 3) && d.kh == d.kw &&
            d.pad == d.kh / 2 && d.Kpitch == d.kh * d.kw * d.Cin && (W == 56 || W == 28 || W == 14 || W == 7);
+}
+
+// Split-K limits.  Weight gradients run on side streams NEXT to the data-gradient chain: a launch owns its SMs (one CTA of 170 KB
+// each), so its K-slices are limited to a CTA budget that leaves room for the chain (DBOA_WGRAD_MAX_CTAS, at least 1).
+// DBOA_WGRAD_MAX_NZ: largest cluster (K-slices of one tile).  A cluster needs that many free SMs inside ONE GPC, so large
+// clusters cannot start next to another stream's kernel that has CTAs in every GPC.
+static int wgrad_budget_default() { const char* e = getenv("DBOA_WGRAD_MAX_CTAS"); return clamp_split(e ? atoi(e) : 128, 1, 1 << 30); }
+static int wgrad_max_nz_default() { const char* e = getenv("DBOA_WGRAD_MAX_NZ"); return clamp_split(e ? atoi(e) : 16, 1, 16); }
+static int g_wgrad_budget = wgrad_budget_default();
+static int g_wgrad_max_nz = wgrad_max_nz_default();
+static int g_wgrad_min_kb = 1;
+void conv_wgrad_wide_set_limits(int max_ctas, int max_nz, int min_kb) {
+    g_wgrad_budget = max_ctas < 0 ? wgrad_budget_default() : clamp_split(max_ctas, 1, 1 << 30);
+    g_wgrad_max_nz = max_nz < 0 ? wgrad_max_nz_default() : clamp_split(max_nz, 1, 16);
+    g_wgrad_min_kb = min_kb < 0 ? 1 : clamp_split(min_kb, 1, 1 << 30);
 }
 
 int conv_wgrad_wide(const float* dy, const float* x, float* dw, const ConvDims& d, cudaStream_t st, bool pdl) {
@@ -319,19 +340,14 @@ int conv_wgrad_wide(const float* dy, const float* x, float* dw, const ConvDims& 
     L.kps = ceil_div(d.Ho, bh); L.nkb_total = d.B * L.kps;
     L.ntn = d.Cin / wg::BN; L.taps = d.kh * d.kw;
     const int tiles = (d.Cout / wg::BM) * L.ntn * L.taps;
-    // weight gradients run on side streams NEXT to the data-gradient chain: a launch owns its SMs (one CTA of 170 KB each), so its
-    // K-slices are limited to a CTA budget that leaves room for the chain (DBOA_WGRAD_MAX_CTAS)
-    static const int budget = [] { const char* e = getenv("DBOA_WGRAD_MAX_CTAS"); int v = e ? atoi(e) : 128; return v < 1 ? 1 : v; }();
     int nz = 1;
-    // DBOA_WGRAD_MAX_NZ: largest cluster (K-slices of one tile).  A cluster needs that many free SMs inside ONE GPC, so large
-    // clusters cannot start next to another stream's kernel that has CTAs in every GPC.
-    static const int max_nz = [] { const char* e = getenv("DBOA_WGRAD_MAX_NZ"); int v = e ? atoi(e) : 16; return v < 1 ? 1 : (v > 16 ? 16 : v); }();
-    while (nz < max_nz && tiles * nz * 2 <= budget && L.nkb_total / (nz * 2) >= 1) nz *= 2;
+    while (nz < g_wgrad_max_nz && tiles * nz * 2 <= g_wgrad_budget && L.nkb_total / (nz * 2) >= g_wgrad_min_kb) nz *= 2;
     while (nz > 1 && (nz - 1) * ceil_div(L.nkb_total, nz) >= L.nkb_total) nz >>= 1;
     L.nz = nz; L.per = ceil_div(L.nkb_total, nz);
     const CUtensorMap* tmdy = static_cast<const CUtensorMap*>(tma_act_map(dy, d.B, d.Ho, d.Wo, d.Cout, W, bh, true, 1));
     const CUtensorMap* tmx = static_cast<const CUtensorMap*>(tma_act_map(x, d.B, d.Hi, d.Wi, d.Cin, W, bh, true, d.stride));
     if (tmdy == nullptr || tmx == nullptr) return DBOA_ERR_CUDA;
+    wide_plan_note(2, nz, L.per, 2, tiles * nz, L.nkb_total);      // two operand stages
     const size_t smem = 4 * (size_t)wg::STAGE + 1024 + 1024;
     return launch_ex(wg::conv_wgrad_wide_kernel, dim3(tiles * nz), dim3(wg::NT), smem, st, dim3(nz, 1, 1), pdl, L, *tmdy, *tmx);
 }

@@ -961,13 +961,22 @@ bool conv_wide_ok(const FusedConv& d) {
 static bool g_operand_tmem = [] { const char* e = getenv("DBOA_OPERAND_TMEM"); return e ? e[0] != '0' : true; }();
 void conv_wide_set_operand_tmem(bool on) { g_operand_tmem = on; }
 bool conv_wide_operand_tmem() { return g_operand_tmem; }
-static int g_cta_budget = [] { const char* e = getenv("DBOA_FUSED_MAX_CTAS"); int v = e ? atoi(e) : 96; return v; }();
+static int fused_cta_budget_default() { const char* e = getenv("DBOA_FUSED_MAX_CTAS"); return e ? atoi(e) : 96; }
+static int fused_min_kb_default() { const char* e = getenv("DBOA_FUSED_MINKB"); return e ? atoi(e) : 2; }
+static int fused_max_nz_default() { const char* e = getenv("DBOA_FUSED_MAX_NZ"); return e ? atoi(e) : 16; }
+static int g_cta_budget = fused_cta_budget_default();
+static int g_min_kb = clamp_split(fused_min_kb_default(), 1, 1 << 30);     // k-blocks a K-slice must at least hold
+static int g_max_nz = clamp_split(fused_max_nz_default(), 1, 16);           // largest cluster (K-slices of one tile)
 void conv_wide_set_cta_budget(int n) { g_cta_budget = n; }
+void conv_wide_set_limits(int max_ctas, int max_nz, int min_kb) {
+    g_cta_budget = max_ctas < 0 ? fused_cta_budget_default() : max_ctas;
+    g_max_nz = clamp_split(max_nz < 0 ? fused_max_nz_default() : max_nz, 1, 16);
+    g_min_kb = clamp_split(min_kb < 0 ? fused_min_kb_default() : min_kb, 1, 1 << 30);
+}
 int conv_wide_plan(const FusedConv* d, int nprob, int B) {
     int tiles = 0;
     for (int i = 0; i < nprob; ++i) tiles += B * ceil_div(d[i].Ho, wz::rows_of(d[i].Ho)) * (d[i].Cout / wz::BN);
     const int nkb = d[0].k * d[0].k * d[0].Cin / wz::BK;
-    static const int min_kb = [] { const char* e = getenv("DBOA_FUSED_MINKB"); int v = e ? atoi(e) : 2; return v < 1 ? 1 : v; }();
     int nz = 1;
     // the budget limits how far a launch with FEW tiles is split; a launch whose tiles alone exceed it (large batches) may still
     // split up to the hardware wave, which halves its accumulation chains
@@ -976,10 +985,21 @@ int conv_wide_plan(const FusedConv* d, int nprob, int B) {
         const int soft = g_cta_budget > 2 * tiles ? g_cta_budget : 2 * tiles;
         return g_cta_budget > 0 && soft < hw ? soft : hw;
     };
-    static const int max_nz = [] { const char* e = getenv("DBOA_FUSED_MAX_NZ"); int v = e ? atoi(e) : 16; return v < 1 ? 1 : (v > 16 ? 16 : v); }();
-    while (nz < max_nz && tiles * nz * 2 <= cap(nz * 2) && nkb / (nz * 2) >= min_kb) nz *= 2;
+    while (nz < g_max_nz && tiles * nz * 2 <= cap(nz * 2) && nkb / (nz * 2) >= g_min_kb) nz *= 2;
     while (nz > 1 && (nz - 1) * ceil_div(nkb, nz) >= nkb) nz >>= 1;
     return nz;
+}
+
+// split-K plan of the most recent launch of each wide kernel (dboa_last_wide_plan): one host store per launch
+static WidePlan g_last_plan[3];
+void wide_plan_note(int kernel, int nz, int per, int D, int grid, int nkb) {
+    g_last_plan[kernel] = WidePlan{nz, per, D, grid, nkb - (nz - 1) * per};
+}
+bool wide_plan_last(int kernel, long long out[5]) {
+    if (kernel < 0 || kernel > 2) return false;
+    const WidePlan& p = g_last_plan[kernel];
+    out[0] = p.nz; out[1] = p.per; out[2] = p.D; out[3] = p.grid; out[4] = p.last;
+    return true;
 }
 
 #ifdef DBOA_TIMELINE
@@ -1035,6 +1055,7 @@ int conv_wide_launch(const FusedConv* d, int nprob, int B, int nz, const float* 
     const size_t smem = fixed + (size_t)D * slot;
     if (smem > 227 * 1024) return DBOA_ERR_SHAPE;
     const dim3 grid(total * nz), block(wz::NT), cl(nz, 1, 1);
+    wide_plan_note(0, nz, per, D, (int)grid.x, nkb);
     if (dep != nullptr) {
         // mode 0 has no statistics barrier behind which the other transform threads could be ordered: every thread waits there
         L.dep_flag = pdl ? dep->wait_flag : nullptr; L.dep_expect = dep->wait_count; L.done_flag = dep->signal_flag;

@@ -718,6 +718,19 @@ bool dgrad_wide_ok(const ConvDims& d) {
            d.pad == d.kh / 2 && d.Kpitch == d.kh * d.kw * d.Cin && d.Hi <= 128;
 }
 
+// split-K limits: CTA budget (DBOA_DGRAD_MAX_CTAS; a budget that does not exceed twice the tiles means 2 x tiles, at most 128),
+// largest cluster (DBOA_DGRAD_MAX_NZ) and the fewest k-blocks a K-slice may hold
+static int dgrad_budget_default() { const char* e = getenv("DBOA_DGRAD_MAX_CTAS"); return e ? atoi(e) : 64; }
+static int dgrad_max_nz_default() { const char* e = getenv("DBOA_DGRAD_MAX_NZ"); return clamp_split(e ? atoi(e) : 16, 1, 16); }
+static int g_dgrad_budget = dgrad_budget_default();
+static int g_dgrad_max_nz = dgrad_max_nz_default();
+static int g_dgrad_min_kb = 2;
+void dgrad_wide_set_limits(int max_ctas, int max_nz, int min_kb) {
+    g_dgrad_budget = max_ctas < 0 ? dgrad_budget_default() : max_ctas;
+    g_dgrad_max_nz = max_nz < 0 ? dgrad_max_nz_default() : clamp_split(max_nz, 1, 16);
+    g_dgrad_min_kb = min_kb < 0 ? 2 : clamp_split(min_kb, 1, 1 << 30);
+}
+
 int dgrad_wide(const DgradFused& f, const ConvDims& d, cudaStream_t st, bool pdl) {
     if (!dgrad_wide_ok(d)) return DBOA_ERR_UNSUPPORTED;
     dz::Launch L;
@@ -732,10 +745,10 @@ int dgrad_wide(const DgradFused& f, const ConvDims& d, cudaStream_t st, bool pdl
     L.bh = d.Hi * d.Hi <= dz::BM ? d.Hi : dz::BM / d.Hi;
     L.tps = ceil_div(d.Hi, L.bh); L.ntiles = d.Cin / dz::BN;
     const int tiles = d.B * L.tps * L.ntiles, nkb = d.kh * d.kw * d.Cout / dz::BK;
-    static const int budget = [] { const char* e = getenv("DBOA_DGRAD_MAX_CTAS"); int v = e ? atoi(e) : 64; return v; }();
+    const int budget = g_dgrad_budget;
     int nz = 1;
-    static const int max_nz = [] { const char* e = getenv("DBOA_DGRAD_MAX_NZ"); int v = e ? atoi(e) : 16; return v < 1 ? 1 : (v > 16 ? 16 : v); }();
-    while (nz < max_nz && tiles * nz * 2 <= (budget > 2 * tiles ? budget : (2 * tiles < 128 ? 2 * tiles : 128)) && nkb / (nz * 2) >= 2) nz *= 2;
+    while (nz < g_dgrad_max_nz && tiles * nz * 2 <= (budget > 2 * tiles ? budget : (2 * tiles < 128 ? 2 * tiles : 128)) && nkb / (nz * 2) >= g_dgrad_min_kb)
+        nz *= 2;
     while (nz > 1 && (nz - 1) * ceil_div(nkb, nz) >= nkb) nz >>= 1;
     L.nz = nz; L.per = ceil_div(nkb, nz);
     L.tabc = d.kh == 1 ? L.per * dz::BK : d.Cout;
@@ -748,6 +761,7 @@ int dgrad_wide(const DgradFused& f, const ConvDims& d, cudaStream_t st, bool pdl
     const CUtensorMap* tmy = static_cast<const CUtensorMap*>(tma_act_map(f.y_c, d.B, d.Hi, d.Wi, d.Cout, d.Wi, L.bh, false, 1));
     const CUtensorMap* tmw = static_cast<const CUtensorMap*>(tma_weight_map_mn(f.w, d.kh * d.kw * d.Cin, d.Cout));
     if (!tmdz || !tmy || !tmw) return DBOA_ERR_CUDA;
+    wide_plan_note(1, nz, L.per, D, tiles * nz, nkb);
     return conv_wide_operand_tmem() ? launch_ex(dz::dgrad_wide_kernel<true>, dim3(tiles * nz), dim3(dz::NT), smem, st, dim3(nz, 1, 1), pdl, L, *tmdz, *tmy, *tmw)
                                     : launch_ex(dz::dgrad_wide_kernel<false>, dim3(tiles * nz), dim3(dz::NT), smem, st, dim3(nz, 1, 1), pdl, L, *tmdz, *tmy, *tmw);
 }

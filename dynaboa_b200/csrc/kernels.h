@@ -46,6 +46,16 @@ struct FusedConv {
 bool conv_wide_ok(const FusedConv& d);
 int conv_wide_plan(const FusedConv* d, int nprob, int B);
 void conv_wide_set_cta_budget(int n);                                  // 0: all SMs
+// split-K limits of the planners (a negative argument restores the environment default; see dboa_set_split_limits)
+void conv_wide_set_limits(int max_ctas, int max_nz, int min_kb);
+void dgrad_wide_set_limits(int max_ctas, int max_nz, int min_kb);
+void conv_wgrad_wide_set_limits(int max_ctas, int max_nz, int min_kb);
+inline int clamp_split(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
+// plan of the most recent launch of kernel 0 (conv_wide), 1 (dgrad_wide), 2 (conv_wgrad_wide): K-slices (= cluster size),
+// k-blocks per slice, operand ring depth, grid size, k-blocks of the last slice
+struct WidePlan { long long nz, per, D, grid, last; };
+void wide_plan_note(int kernel, int nz, int per, int D, int grid, int nkb);
+bool wide_plan_last(int kernel, long long out[5]);
 int map_cache_selftest(int bound, int n, int window);                   // host-only check of the tensor-map cache's eviction rule
 void conv_wide_set_operand_tmem(bool on);                              // transformed activation operand of conv_wide / dgrad_wide in tensor memory
 bool conv_wide_operand_tmem();

@@ -45,6 +45,18 @@ int dboa_set_fused_backward(int enable);
 /* CTAs (= SMs) the fused convolutions of the following dboa_hmr_forward calls may use; 0 = all.  Forwards issued side by side
  * on different streams share the device when each is given about half of it (a fused launch owns its SMs). */
 int dboa_set_forward_cta_budget(int n);
+/* Split-K limits of the planner of one tcgen05 kernel -- kernel 0: fused convolution (csrc/conv_wide.cu), 1: fused data gradient
+ * (csrc/dgrad_wide.cu), 2: weight gradient (csrc/conv_wgrad_wide.cu).  A launch splits the reduction of a tile into nz K-slices
+ * (nz = thread-block cluster size, a power of two <= max_nz) while the launch stays within max_ctas CTAs and every slice keeps at
+ * least min_kb k-blocks.  A negative argument restores that limit's default (environment: DBOA_FUSED_MAX_CTAS / _MAX_NZ / _MINKB
+ * for kernel 0, DBOA_DGRAD_MAX_CTAS / _MAX_NZ for 1, DBOA_WGRAD_MAX_CTAS / _MAX_NZ for 2; min_kb 2, 2, 1).  max_ctas = 0 does
+ * not mean the same for every kernel: kernel 0 takes it as "every SM" (as dboa_set_forward_cta_budget), kernel 1 as "twice the
+ * tiles, at most 128", kernel 2 clamps it to 1 (no split).  Kernel 0's max_ctas is the budget dboa_set_forward_cta_budget sets.
+ * Returns DBOA_ERR_ARG for another kernel index. */
+int dboa_set_split_limits(int kernel, int max_ctas, int max_nz, int min_kb);
+/* Plan of the most recent launch of `kernel` (indices as above) in this process: out = {nz, k-blocks per slice, operand ring
+ * depth, grid size in CTAs, k-blocks of the last slice}; all zero before the first launch.  DBOA_ERR_ARG for another index. */
+int dboa_last_wide_plan(int kernel, long long out[5]);
 /* 1: the fused convolution / data-gradient kernels keep the transformed activation operand (TF32 hi and lo parts) in tensor
  * memory and the tensor core reads only the weight operand from shared memory; 0: both operands in shared memory (the A/B
  * reference of the same kernels).  Same results to fp32 rounding of the same products (the split is identical).

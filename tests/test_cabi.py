@@ -62,6 +62,14 @@ def test_argument_errors_do_not_need_a_gpu(lib):
     off, nd = ctypes.c_longlong(), ctypes.c_int()
     shp, st = (ctypes.c_longlong * 4)(), (ctypes.c_longlong * 4)()
     assert lib.dboa_hmr_param_info(999, None, 0, ctypes.byref(off), ctypes.byref(nd), shp, st) == -1
+    plan = (ctypes.c_longlong * 5)()
+    for kernel in (-1, 3):
+        assert lib.dboa_last_wide_plan(kernel, plan) == -1
+        assert lib.dboa_set_split_limits(kernel, -1, -1, -1) == -1
+    assert lib.dboa_last_wide_plan(0, None) == -1
+    for kernel in (0, 1, 2):
+        assert lib.dboa_last_wide_plan(kernel, plan) == 0
+        assert lib.dboa_set_split_limits(kernel, -1, -1, -1) == 0      # restore the defaults: changes nothing here
 
 
 def test_tensor_map_cache_keeps_held_pointers_across_evictions(lib):
